@@ -54,7 +54,15 @@ def parse_args():
                     help="train: the headline training step; dscnn: DS-CNN-S forward (BASELINE.json config 5, comparison point); "
                          "infer: evaluation-mode forward from wav (config 1 with --batch 1: latency); "
                          "augment: the device input stage (SURVEY.md 8f row 1), an HBM-bound elementwise pass")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (float32), so that two "
+                         "builds can be compared output for output (the inputs are seeded: the same arguments give the same inputs)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
+    return a
 
 
 def l2_policy(a, clip=16000):
@@ -97,6 +105,22 @@ def pin_to_gpu_numa_node(dev_index):
     except Exception:
         return None
     return None
+
+
+DUMP_ELEMENTS = 15_000_000          # 60 MB of float32 over all dumped arrays
+
+
+def dump_outputs(path, arrays):
+    """Writes {name: tensor} as path/<name>.npy in float32.  An array larger than its even share of DUMP_ELEMENTS is replaced by a
+    fixed, seeded sample of its elements (flattened, in index order): the same elements on every run with the same arguments."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    cap = DUMP_ELEMENTS // len(arrays)
+    for name, t in arrays.items():
+        x = t.detach().float().cpu().numpy()
+        if x.size > cap:
+            x = x.ravel()[np.sort(np.random.default_rng(0).choice(x.size, cap, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), x)
 
 
 def workload_name(a):
@@ -344,6 +368,8 @@ def run_ours(a):
         step(i)
     e1.record()
     barrier()
+    if a.dump_outputs and rank == 0:      # now: the end-to-end and per-kernel passes below keep training the same variables
+        dump_outputs(a.dump_outputs, {"losses": losses, "params": params, "slots": slots, "moving": moving})
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
     if world > 1:
         torch.distributed.all_reduce(ms, op=torch.distributed.ReduceOp.MAX)
@@ -399,7 +425,7 @@ def run_ours(a):
         from tcresnet_b200.engine import HostFeed
         h_wavs = [w.cpu().pin_memory() for w in wavs[:min(rot, 4)]]
         h_hots = [o.cpu().pin_memory() for o in onehots[:min(rot, 4)]]
-        esteps = max(100, min(a.steps, 200))            # never fewer than 100 timed steps, whatever --steps says
+        esteps = a.steps
 
         def e2e_run(host_wavs, host_clips=None, background=None):
             feed = HostFeed(eng, lag=2)
@@ -647,9 +673,11 @@ def run_infer(a):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(a.steps):
-        eng.forward(wavs[i % a.rotate], params, moving)
+        res = eng.forward(wavs[i % a.rotate], params, moving)
     e1.record()
     torch.cuda.synchronize()
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, {"logits": res["logits"], "probs": res["probs"]})
     ms = e0.elapsed_time(e1) / a.steps
     h_wav = wavs[0].cpu().pin_memory()
     d_wav = torch.empty_like(wavs[0])
@@ -692,6 +720,8 @@ def run_augment(a):
         eng.augment(pcm[i % rot], clips[i % rot], background, out=outs[i % rot])
     e1.record()
     torch.cuda.synchronize()
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, {"wav": outs[(a.steps - 1) % rot]})
     ms = e0.elapsed_time(e1) / a.steps
     peaks = {}
     try:
@@ -731,9 +761,11 @@ def run_dscnn(a):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(a.steps):
-        net.forward(feats[i % a.rotate], params)
+        logits, probs = net.forward(feats[i % a.rotate], params)
     e1.record()
     torch.cuda.synchronize()
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, {"logits": logits, "probs": probs})
     ms = e0.elapsed_time(e1)
     value = n * a.steps / (ms * 1e-3)
     # per-kernel durations (separate pass: the event brackets add overhead) and the roofline of the dominant kernel
@@ -785,7 +817,7 @@ def run_dscnn(a):
     h_feats = [f.cpu().pin_memory() for f in feats[:4]]
     d_in = torch.empty(n, 49, 40, device=dev)
     h_out = torch.empty(n, 12).pin_memory()
-    esteps = max(100, min(a.steps, 200))
+    esteps = a.steps
     for i in range(12):
         d_in.copy_(h_feats[i % 4], non_blocking=True)
         h_out.copy_(net.forward(d_in, params)[1], non_blocking=True)
