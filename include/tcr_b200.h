@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define TCR_ABI_VERSION 5
+#define TCR_ABI_VERSION 6
 
 enum {
   TCR_OK = 0,
@@ -126,7 +126,7 @@ typedef struct tcr_step_args {
   float*       logits;       /* optional device [n, num_classes] */
   float*       probs;        /* optional device [n, num_classes] softmax (output/softmax) */
   float*       grads;        /* optional device [num_trainable]: gradient of total_loss actually applied */
-  int32_t      apply_update; /* 1: momentum update + BN moving update; 0: gradients only */
+  int32_t      apply_update; /* 1: optimizer update (+ EMA) + BN moving update; 0: gradients only */
   /* Optional device input stage in front of the front-end (TCR_INPUT_WAV_PCM16 only, see tcr_augment_pcm16): when `clips` is not
    * NULL, `input` holds the wav files' int16 samples [n, pcm_stride] and the step first decodes / shifts / mixes / clips them
    * into an internal fp32 buffer.  Zero-initialise these fields when the stage is not used. */
@@ -139,7 +139,31 @@ typedef struct tcr_step_args {
    * the rest of the step waits for it on `stream`.  0: everything is ordered on `stream` (the default; zero-initialise).
    * tcr_train_step_host sets it itself: its inputs arrive on the library's copy stream. */
   int32_t      input_resident;
+  /* Update rule (ABI v6; helper/trainer.py:171-197 build_optimizer).  A zero-initialised tail is today's momentum step.
+   *   TCR_OPT_MOMENTUM  tf.train.MomentumOptimizer: slots = `<var>/Momentum`; `momentum` 0 is GradientDescentOptimizer.
+   *   TCR_OPT_ADAM      tf.train.AdamOptimizer: slots = m (`<var>/Adam`, init 0), slots2 = v (`<var>/Adam_1`, init 0),
+   *                     opt_scalars = device [2] {beta1_power, beta2_power} (init beta1, beta2).  Per element, in fp32:
+   *                     alpha = lr*sqrt(1-beta2_power)/(1-beta1_power); m += (g-m)*(1-beta1); v += (g^2-v)*(1-beta2);
+   *                     w -= m*alpha/(sqrt(v)+epsilon).  The powers are multiplied by beta1 / beta2 once per applied step,
+   *                     inside the update launch (the caller owns the buffer, so CUDA-graph replays advance it as well).
+   *   TCR_OPT_RMSPROP   tf.train.RMSPropOptimizer, not centered: slots = ms (`<var>/RMSProp`, init ONES), slots2 = mom
+   *                     (`<var>/RMSProp_1`, init 0): ms += (g^2-ms)*(1-rms_decay); mom = mom*momentum + g*lr/sqrt(ms+epsilon);
+   *                     w -= mom.
+   * g is the gradient `grads` reports: weight decay included (L2 in the loss, not AdamW), averaged over ranks.
+   * ema != NULL: tf.train.ExponentialMovingAverage(ema_decay).apply(trainables) after the update (helper/trainer.py:213-217):
+   * shadow -= (shadow - w) * (1 - ema_decay), on the updated weights, fixed decay; the shadow (`<var>/ExponentialMovingAverage`)
+   * starts as a copy of the initial weights.  apply_update == 0 changes none of this state. */
+  int32_t      optimizer;    /* TCR_OPT_* */
+  float*       slots2;       /* flat [num_trainable]: Adam v / RMSProp mom; NULL for momentum */
+  float*       opt_scalars;  /* device [2]: Adam beta1_power, beta2_power; NULL otherwise */
+  float        beta1;        /* 0.9 */
+  float        beta2;        /* 0.999 */
+  float        epsilon;      /* Adam 1e-8, RMSProp 1e-10 */
+  float        rms_decay;    /* 0.9 */
+  float*       ema;          /* flat [num_trainable] EMA shadows, or NULL: no EMA */
+  float        ema_decay;    /* 0.999 */
 } tcr_step_args;
+enum { TCR_OPT_MOMENTUM = 0, TCR_OPT_ADAM = 1, TCR_OPT_RMSPROP = 2 };
 
 int         tcr_abi_version(void);
 const char* tcr_last_error(void);
@@ -210,9 +234,9 @@ int tcr_forward(tcr_handle* h, const float* input, int32_t input_is_features, co
 int tcr_eval_accumulate(tcr_handle* h, const float* scores, const float* onehot, int32_t n, int32_t topk, int64_t* counts,
                         tcr_stream stream);
 
-/* Forward + backward + SGD-momentum + BN moving-average update (helper/trainer.py:171-222,
- * slim.learning.create_train_op).  With a communicator attached (tcr_comm_init) gradients are
- * averaged over ranks with one ncclAllReduce before the update. */
+/* Forward + backward + optimizer update (momentum / Adam / RMSProp, optional EMA; see tcr_step_args::optimizer) + BN
+ * moving-average update (helper/trainer.py:171-222, slim.learning.create_train_op).  With a communicator attached
+ * (tcr_comm_init) gradients are averaged over ranks with one ncclAllReduce before the update. */
 int tcr_train_step(tcr_handle* h, const tcr_step_args* args, tcr_stream stream);
 
 /* The same step fed from PINNED HOST memory (the feed_dict / tf.data side of session.run(train_op): helper/trainer.py:312-321,

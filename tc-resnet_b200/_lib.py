@@ -14,8 +14,9 @@ LIB_PATH = os.path.join(_HERE, "libtcr_b200.so")
 
 TCR_MODEL_TCRESNET8 = 8
 TCR_MODEL_TCRESNET14 = 14
-ABI_VERSION = 5          # TCR_ABI_VERSION of include/tcr_b200.h this binding was written against
+ABI_VERSION = 6          # TCR_ABI_VERSION of include/tcr_b200.h this binding was written against
 TCR_INPUT_WAV_F32, TCR_INPUT_FEATURES, TCR_INPUT_WAV_PCM16 = 0, 1, 2
+TCR_OPT_MOMENTUM, TCR_OPT_ADAM, TCR_OPT_RMSPROP = 0, 1, 2
 TCR_FEATURE_MFCC = 0
 TCR_FEATURE_LOG_MEL = 1
 KIND_NAMES = {0: "weight", 1: "beta", 2: "gamma", 3: "moving_mean", 4: "moving_variance"}
@@ -69,6 +70,9 @@ class TcrStepArgs(C.Structure):
         ("dropout_seed", C.c_uint64), ("dropout_mask", C.c_void_p), ("losses", C.c_void_p),
         ("logits", C.c_void_p), ("probs", C.c_void_p), ("grads", C.c_void_p), ("apply_update", C.c_int32),
         ("clips", C.c_void_p), ("background", C.c_void_p), ("pcm_stride", C.c_int64), ("input_resident", C.c_int32),
+        # ABI v6: update rule (zero = momentum, as before)
+        ("optimizer", C.c_int32), ("slots2", C.c_void_p), ("opt_scalars", C.c_void_p), ("beta1", C.c_float),
+        ("beta2", C.c_float), ("epsilon", C.c_float), ("rms_decay", C.c_float), ("ema", C.c_void_p), ("ema_decay", C.c_float),
     ]
 
 

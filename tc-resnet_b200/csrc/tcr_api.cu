@@ -643,11 +643,27 @@ static void frontend_ahead_destroy(tcr_handle* h) {
 #endif
 }
 
+// The state buffers each update rule reads and writes (tcr_step_args::optimizer).
+static int check_optimizer(const tcr_step_args* a) {
+  switch (a->optimizer) {
+    case TCR_OPT_MOMENTUM: break;
+    case TCR_OPT_ADAM:
+      if (a->apply_update && (!a->slots2 || !a->opt_scalars)) return fail(TCR_ERR_INVALID, "TCR_OPT_ADAM needs slots2 (v) and opt_scalars (beta powers)");
+      break;
+    case TCR_OPT_RMSPROP:
+      if (a->apply_update && !a->slots2) return fail(TCR_ERR_INVALID, "TCR_OPT_RMSPROP needs slots2 (mom)");
+      break;
+    default: return fail(TCR_ERR_INVALID, "unknown optimizer %d", a->optimizer);
+  }
+  return TCR_OK;
+}
+
 // input_event: what the front-end has to wait for when it runs ahead (the host feed's H2D copy), or null
 static int train_step_impl(tcr_handle* h, const tcr_step_args* a, tcr_stream stream, void* input_event) {
   pdl_chain_reset();
   if (!h || !a || !a->input || !a->onehot || !a->params) return fail(TCR_ERR_INVALID, "NULL argument");
   if (a->apply_update && (!a->slots || !a->moving)) return fail(TCR_ERR_INVALID, "apply_update needs slots and moving");
+  TCR_TRY(check_optimizer(a));
   TCR_TRY(check_n(h, a->n));
   cudaStream_t s = (cudaStream_t)stream;
   const float* feat = a->input;
@@ -801,6 +817,7 @@ extern "C" int tcr_train_step_host(tcr_handle* h, const tcr_step_args* a, int32_
                                    int64_t* losses_step) {
   if (!h || !a || !a->input || !a->onehot || !a->params) return fail(TCR_ERR_INVALID, "NULL argument");
   if (lag < 0 || lag >= kFeedDepth) return fail(TCR_ERR_INVALID, "lag must be in [0, %d]", kFeedDepth - 1);
+  TCR_TRY(check_optimizer(a));       // before anything is queued; the struct copy below carries the optimizer fields to the step
   TCR_TRY(check_n(h, a->n));
   HostFeedState* f = nullptr;
   TCR_TRY(hostfeed_get(h, &f));

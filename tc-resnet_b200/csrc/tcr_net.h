@@ -34,7 +34,8 @@ int net_weight_gradients(tcr_handle* h, const float* feat, int n, cudaStream_t s
 void resident_destroy(tcr_handle* h);
 int net_backward(tcr_handle* h, const float* feat, const float* params, int n, cudaStream_t s);
 
-// Gradient finalisation (+ weight decay), optional NCCL all-reduce, momentum update, BN moving averages, losses.
+// Gradient finalisation (+ weight decay), optional NCCL all-reduce, optimizer update (tcr_step_args::optimizer, + EMA), BN moving
+// averages, losses.
 int net_update(tcr_handle* h, const float* feat, const tcr_step_args* a, cudaStream_t s);
 
 int launch_loss_only(tcr_handle* h, const float* params, float weight_decay, int n, float* losses, cudaStream_t s);

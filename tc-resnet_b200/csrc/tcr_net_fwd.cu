@@ -612,6 +612,7 @@ int net_alloc_workspace(tcr_handle* h) {
   WS(ws_alloc(h, &h->d_hyper, 1));
   WS(ws_alloc(h, &h->d_gridbar, 64));
   cudaMemset(h->d_gridbar, 0, 64 * sizeof(unsigned));
+  h->d_opt_ticket = h->d_gridbar + 32;     // the resident grid barrier uses word 0; the ticket gets its own 128-byte line
   if (getenv("TCR_DEBUG_TIMELINE")) {
     WS(ws_alloc(h, &h->d_timeline, (size_t)16 * 8192));
     cudaMemset(h->d_timeline, 0, sizeof(long long) * 16 * 8192);

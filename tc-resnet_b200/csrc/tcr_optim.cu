@@ -1,11 +1,13 @@
-// tcr_optim.cu — gradient finalisation, SGD-momentum update, BN moving averages, loss scalars.
+// tcr_optim.cu — gradient finalisation, optimizer update (momentum / Adam / RMSProp, EMA), BN moving averages, loss scalars.
 //
 // Replaces, per training step: the 12/18 L2Loss nodes + AddN (factory/audio_nets.py:175-182), the 32/50
-// per-variable ApplyMomentum nodes (tf.train.MomentumOptimizer, helper/trainer.py:188-190: m <- mom*m + g;
-// v <- v - lr*m) and the 20/32 AssignSub moving-average updates of slim.batch_norm (decay 0.997, UNBIASED
-// batch variance, no zero-debias) with two flat multi-tensor kernels over the parameter buffer:
-//   grad_finalize_kernel : g[p] = sum_r partial[r][p] (+ weight_decay * w[p]); per-block sum of w^2
-//   update_kernel        : m <- mom*m + g/world ; w <- w - lr*m ; moving stats ; loss scalars
+// per-variable ApplyMomentum / ApplyAdam / ApplyRMSProp nodes (helper/trainer.py:171-197; Adam's _finish advancing the beta
+// powers), the ExponentialMovingAverage of --use_ema (:213-217) and the 20/32 AssignSub moving-average updates of
+// slim.batch_norm (decay 0.997, UNBIASED batch variance, no zero-debias) with two flat multi-tensor kernels over the parameter
+// buffer:
+//   grad_finalize_kernel       : g[p] = sum_r partial[r][p] (+ weight_decay * w[p]); per-block sum of w^2
+//   update_kernel<rule, ema>   : g/world -> the rule's slots and w (momentum: m <- mom*m + g ; w <- w - lr*m) ; EMA shadow ;
+//                                moving stats ; loss scalars
 // The NCCL all-reduce of the flat gradient sits between the two when a communicator is attached.
 #include "tcr_bn.cuh"
 #include "tcr_net.h"
@@ -85,10 +87,19 @@ __global__ void __launch_bounds__(kOptThreads) grad_finalize_kernel(GradArgs a) 
   grad_finalize_body(a, (int)blockIdx.x, s_red);
 }
 
+// Update rule of update_kernel (template parameter; values of tcr_step_args::optimizer)
+constexpr int kRuleMomentum = TCR_OPT_MOMENTUM, kRuleAdam = TCR_OPT_ADAM, kRuleRmsprop = TCR_OPT_RMSPROP;
+
 struct UpdateArgs {
   int64_t total;
   float* params; float* slots; const float* grads; float* moving;
   float lr, momentum, weight_decay, one_minus_decay, grad_scale;
+  // Adam / RMSProp / EMA (tcr_step_args fields of the same names)
+  float* slots2;          // Adam v, RMSProp mom
+  float* opt_scalars;     // Adam: device [2] beta1_power, beta2_power; advanced by the last CTA to retire
+  unsigned* ticket;       // Adam: retirement counter of this launch, reset by the last CTA
+  float one_minus_beta1, one_minus_beta2, beta1, beta2, epsilon, one_minus_rms_decay;
+  float* ema; float one_minus_ema_decay;
   const MovingSegment* msegs; int nmsegs; int n;
   const float* l2part; int l2blocks;
   const float* ce_sum; int ce_count; float inv_n;      // cross-entropy records of the head launch
@@ -121,6 +132,7 @@ __device__ __forceinline__ unsigned ld_acquire_sys(const unsigned* p) {
 #endif
 }
 
+template <int RULE, bool EMA>
 __global__ void __launch_bounds__(kOptThreads) update_kernel(UpdateArgs a) {
   pdl_wait();
   if (a.p2p_world > 1) {
@@ -151,9 +163,32 @@ __global__ void __launch_bounds__(kOptThreads) update_kernel(UpdateArgs a) {
     const float g = gsum * a.grad_scale;
     if (a.grads_out) a.grads_out[p] = g;
     if (a.apply) {
-      const float m = fmaf(a.slots[p], a.momentum, g);     // accum = accum * momentum + grad
-      a.slots[p] = m;
-      a.params[p] = a.params[p] - a.lr * m;                // var -= lr * accum
+      float w;
+      if (RULE == kRuleMomentum) {                           // ApplyMomentum
+        const float m = fmaf(a.slots[p], a.momentum, g);     // accum = accum * momentum + grad
+        a.slots[p] = m;
+        w = a.params[p] - a.lr * m;                          // var -= lr * accum
+      } else if (RULE == kRuleAdam) {                        // ApplyAdam, in its order
+        const float alpha = a.lr * sqrtf(1.f - a.opt_scalars[1]) / (1.f - a.opt_scalars[0]);
+        float m = a.slots[p], v = a.slots2[p];
+        m += (g - m) * a.one_minus_beta1;
+        v += (g * g - v) * a.one_minus_beta2;
+        a.slots[p] = m;
+        a.slots2[p] = v;
+        w = a.params[p] - (m * alpha) / (sqrtf(v) + a.epsilon);
+      } else {                                               // ApplyRMSProp (not centered)
+        float ms = a.slots[p];
+        ms += (g * g - ms) * a.one_minus_rms_decay;
+        const float mom = a.slots2[p] * a.momentum + (g * a.lr) / sqrtf(ms + a.epsilon);
+        a.slots[p] = ms;
+        a.slots2[p] = mom;
+        w = a.params[p] - mom;
+      }
+      a.params[p] = w;
+      if (EMA) {                                             // ExponentialMovingAverage.apply on the updated weights
+        const float s = a.ema[p];
+        a.ema[p] = s - (s - w) * a.one_minus_ema_decay;
+      }
     }
   }
   // extra CTAs past the parameter range: one per BN layer (moving averages) + one for the loss scalars, so no
@@ -192,6 +227,20 @@ __global__ void __launch_bounds__(kOptThreads) update_kernel(UpdateArgs a) {
       const float model = (float)s_tot[1] * a.inv_n;
       a.losses[1] = model;
       a.losses[0] = model + a.weight_decay * (float)(0.5 * s_tot[0]);
+    }
+  }
+  if (RULE == kRuleAdam && a.apply) {
+    // _finish: beta powers advance once per applied step, after every CTA has read them.  The CTAs are unordered, so the last
+    // one to retire does it (threadFenceReduction pattern) and re-arms the counter for the next launch: no extra launch, and
+    // a CUDA-graph replay advances them too.
+    __syncthreads();                 // every thread of this CTA is past its read of opt_scalars
+    if (threadIdx.x == 0) {
+      __threadfence();
+      if (atomicAdd(a.ticket, 1u) == gridDim.x - 1) {
+        a.opt_scalars[0] = a.opt_scalars[0] * a.beta1;
+        a.opt_scalars[1] = a.opt_scalars[1] * a.beta2;
+        *a.ticket = 0u;
+      }
     }
   }
 }
@@ -286,7 +335,20 @@ int net_update(tcr_handle* h, const float* feat, const tcr_step_args* a, cudaStr
   u.ce_sum = h->d_loss_part; u.ce_count = h->loss_gc; u.inv_n = 1.0f / (float)a->n;
   u.losses = a->losses; u.grads_out = a->grads; u.apply = a->apply_update ? 1 : 0;
   u.param_blocks = blocks;
-  TCR_LAUNCH("update", update_kernel, dim3(blocks + h->n_msegs + 1), dim3(kOptThreads), 0, s, u);
+  // Adam / RMSProp / EMA: TF subtracts the decays from 1 in fp32 (exact for the usual values)
+  u.slots2 = a->slots2; u.opt_scalars = a->opt_scalars; u.ticket = h->d_opt_ticket;
+  u.beta1 = a->beta1; u.beta2 = a->beta2;
+  u.one_minus_beta1 = 1.f - a->beta1; u.one_minus_beta2 = 1.f - a->beta2;
+  u.epsilon = a->epsilon; u.one_minus_rms_decay = 1.f - a->rms_decay;
+  u.ema = a->ema; u.one_minus_ema_decay = 1.f - a->ema_decay;
+  const bool ema = a->ema != nullptr;
+  void (*kfn)(UpdateArgs);
+  switch (a->optimizer) {
+    case TCR_OPT_ADAM: kfn = ema ? update_kernel<kRuleAdam, true> : update_kernel<kRuleAdam, false>; break;
+    case TCR_OPT_RMSPROP: kfn = ema ? update_kernel<kRuleRmsprop, true> : update_kernel<kRuleRmsprop, false>; break;
+    default: kfn = ema ? update_kernel<kRuleMomentum, true> : update_kernel<kRuleMomentum, false>; break;
+  }
+  TCR_LAUNCH("update", kfn, dim3(blocks + h->n_msegs + 1), dim3(kOptThreads), 0, s, u);
   return 0;
 }
 

@@ -100,5 +100,6 @@ struct tcr_handle {
   void* resident = nullptr;          // ResidentState (tcr_resident.cu): layout + program of the resident forward kernel
   int fc_records = 0;                // per-CTA records of the fc weight gradient left by the last head launch
   unsigned* d_gridbar = nullptr;    // arrival counter of the resident kernel's grid barrier (monotonic, never reset)
+  unsigned* d_opt_ticket = nullptr; // retirement counter of the Adam update launch (0 between launches; the last CTA resets it)
   long long* d_timeline = nullptr;   // TCR_DEBUG_TIMELINE=1: per-CTA phase stamps (fwd kernels: 8 slots per CTA; dw: after)
 };

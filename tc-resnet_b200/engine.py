@@ -8,6 +8,7 @@ There is no CPU path: constructing an Engine without a CUDA device or without li
 from __future__ import annotations
 
 import ctypes as C
+from dataclasses import dataclass
 from typing import Dict, Optional
 
 import numpy as np
@@ -17,6 +18,66 @@ from . import _lib as L
 
 _MODELS = {"TCResNet8": 8, "TCResNet8Model": 8, "TCResNet14": 14, "TCResNet14Model": 14, 8: 8, 14: 14}
 _FEATURES = {"mfcc": L.TCR_FEATURE_MFCC, "log_mel_spectrogram": L.TCR_FEATURE_LOG_MEL}
+_RULES = {"mom": L.TCR_OPT_MOMENTUM, "gd": L.TCR_OPT_MOMENTUM, "adam": L.TCR_OPT_ADAM, "rmsprop": L.TCR_OPT_RMSPROP}
+
+
+@dataclass
+class Optimizer:
+    """The update rule of a training step and its hyper-parameters (what helper/trainer.py:build_optimizer chose).
+    kind: "mom" (tf.train.MomentumOptimizer), "gd" (momentum 0), "adam" (tf.train.AdamOptimizer) or "rmsprop"
+    (tf.train.RMSPropOptimizer, not centered).  ema_decay not None: tf.train.ExponentialMovingAverage after every step
+    (--use_ema).  The defaults are TF 1.13's."""
+    kind: str = "mom"
+    momentum: float = 0.9          # mom; rmsprop (default 0.0 there, see rmsprop())
+    beta1: float = 0.9
+    beta2: float = 0.999
+    epsilon: float = 1e-8          # adam 1e-8, rmsprop 1e-10
+    decay: float = 0.9             # rmsprop
+    ema_decay: Optional[float] = None
+
+    def __post_init__(self):
+        if self.kind not in _RULES:
+            raise NotImplementedError(f"optimizer {self.kind!r}")
+
+    @classmethod
+    def rmsprop(cls, decay=0.9, momentum=0.0, epsilon=1e-10, ema_decay=None):
+        return cls("rmsprop", momentum=momentum, epsilon=epsilon, decay=decay, ema_decay=ema_decay)
+
+    @classmethod
+    def adam(cls, beta1=0.9, beta2=0.999, epsilon=1e-8, ema_decay=None):
+        return cls("adam", beta1=beta1, beta2=beta2, epsilon=epsilon, ema_decay=ema_decay)
+
+
+@dataclass
+class OptimizerState:
+    """Device buffers of an update rule, by role.  slots: `<var>/Momentum` | `<var>/Adam` (m) | `<var>/RMSProp` (ms);
+    slots2: `<var>/Adam_1` (v) | `<var>/RMSProp_1` (mom); scalars: [beta1_power, beta2_power] (Adam);
+    ema: `<var>/ExponentialMovingAverage` shadows.  Unused roles are None."""
+    slots: torch.Tensor
+    slots2: Optional[torch.Tensor] = None
+    scalars: Optional[torch.Tensor] = None
+    ema: Optional[torch.Tensor] = None
+
+
+def _set_rule(a: "L.TcrStepArgs", ptr, slots, momentum: float, optimizer: Optional[Optimizer], state: Optional[OptimizerState]):
+    """Fills the update-rule fields of tcr_step_args.  optimizer None: the momentum step with `momentum` (the v5 call)."""
+    opt = optimizer if optimizer is not None else Optimizer("mom", momentum=momentum)
+    if slots is None:
+        if state is None:
+            raise ValueError("train step needs `slots` or an OptimizerState")
+        slots = state.slots
+    a.slots = ptr(slots)
+    a.optimizer = _RULES[opt.kind]
+    a.momentum = 0.0 if opt.kind in ("gd", "adam") else float(opt.momentum)
+    if opt.kind in ("adam", "rmsprop"):
+        if state is None or state.slots2 is None or (opt.kind == "adam" and state.scalars is None):
+            raise ValueError(f"optimizer {opt.kind!r} needs its OptimizerState (Engine.new_optimizer_state)")
+        a.slots2, a.opt_scalars = ptr(state.slots2), ptr(state.scalars)
+        a.beta1, a.beta2, a.epsilon, a.rms_decay = float(opt.beta1), float(opt.beta2), float(opt.epsilon), float(opt.decay)
+    if opt.ema_decay is not None:
+        if state is None or state.ema is None:
+            raise ValueError("EMA needs the shadow buffer of an OptimizerState (Engine.new_optimizer_state)")
+        a.ema, a.ema_decay = ptr(state.ema), float(opt.ema_decay)
 
 
 class Engine:
@@ -115,6 +176,25 @@ class Engine:
                                                       seed, self._stream), "tcr_init_variables")
         return params, slots, moving
 
+    def new_optimizer_state(self, optimizer: Optimizer, params: torch.Tensor, slots: Optional[torch.Tensor] = None) -> OptimizerState:
+        """The state `optimizer` starts from, as TF initialises it: momentum accumulators, Adam m / v at zero and the beta powers at
+        beta1 / beta2, RMSProp ms at ONES and mom at zero, EMA shadows a copy of `params`.  `slots` (e.g. from new_variables) is
+        reused as the first slot buffer when given."""
+        n = params.numel()
+        new = lambda v: torch.full((n,), float(v), dtype=torch.float32, device=params.device)
+        first = slots if slots is not None else new(0.0)
+        st = OptimizerState(slots=first)
+        if optimizer.kind == "adam":
+            first.zero_()
+            st.slots2 = new(0.0)
+            st.scalars = torch.tensor([optimizer.beta1, optimizer.beta2], dtype=torch.float32, device=params.device)
+        elif optimizer.kind == "rmsprop":
+            first.fill_(1.0)
+            st.slots2 = new(0.0)
+        if optimizer.ema_decay is not None:
+            st.ema = params.detach().clone()
+        return st
+
     def variables_to_dict(self, params: torch.Tensor, moving: Optional[torch.Tensor] = None) -> Dict[str, np.ndarray]:
         """{TF variable name: ndarray} — the reference's `var_names_to_values` form (helper/trainer.py:145-154)."""
         p = params.detach().cpu().numpy()
@@ -191,8 +271,11 @@ class Engine:
                    dropout_seed: int = 0, dropout_mask: Optional[torch.Tensor] = None, input_is_features: bool = False,
                    want_outputs: bool = False, want_grads: bool = False, apply_update: bool = True,
                    losses: Optional[torch.Tensor] = None, clips: Optional[torch.Tensor] = None,
-                   background: Optional[torch.Tensor] = None, input_resident: bool = False):
-        """clips (uint8 CUDA tensor of n packed tcr_augment_clip records) + int16 `inputs` [n, stride]: the step starts with
+                   background: Optional[torch.Tensor] = None, input_resident: bool = False,
+                   optimizer: Optional[Optimizer] = None, state: Optional[OptimizerState] = None):
+        """optimizer / state: the update rule and its buffers (new_optimizer_state); without them the step is SGD-momentum with
+        `momentum` on `slots`.  With a state, `slots` may be None (state.slots is used).
+        clips (uint8 CUDA tensor of n packed tcr_augment_clip records) + int16 `inputs` [n, stride]: the step starts with
         the device input stage (decode, shift, background mix, clip) instead of taking decoded fp32 samples.
         input_resident=True: `inputs` is final when the call is made (nothing queued on the current stream writes it); the
         front-end then runs ahead on the library's own stream and overlaps the previous step's tail (tcr_step_args::input_resident)."""
@@ -205,8 +288,9 @@ class Engine:
         else:
             a.input, a.input_is_features = self._input(inputs, input_is_features)
         a.onehot, a.n = self._ptr(onehot), n
-        a.params, a.slots, a.moving = self._ptr(params), self._ptr(slots), self._ptr(moving)
-        a.learning_rate, a.momentum, a.weight_decay = float(learning_rate), float(momentum), float(weight_decay)
+        a.params, a.moving = self._ptr(params), self._ptr(moving)
+        _set_rule(a, self._ptr, slots, momentum, optimizer, state)
+        a.learning_rate, a.weight_decay = float(learning_rate), float(weight_decay)
         a.dropout_seed, a.dropout_mask = int(dropout_seed), self._ptr(dropout_mask)
         losses = losses if losses is not None else self._f32(2)
         out = dict(losses=losses)
@@ -320,10 +404,11 @@ class HostFeed:
 
     def submit(self, h_inputs: torch.Tensor, h_onehot: torch.Tensor, params, slots, moving, learning_rate, momentum=0.9,
                weight_decay=1e-4, dropout_seed=0, input_is_features=False, h_clips: Optional[torch.Tensor] = None,
-               background: Optional[torch.Tensor] = None):
+               background: Optional[torch.Tensor] = None, optimizer: Optional[Optimizer] = None,
+               state: Optional[OptimizerState] = None):
         """h_clips (pinned uint8 tensor of n packed tcr_augment_clip records, datasets/device_input_stage.py) with int16
         h_inputs [n, stride]: the wav files' samples and the per-clip draws cross the bus; the input stage runs on the device
-        (`background`: the CUDA-resident bank)."""
+        (`background`: the CUDA-resident bank).  optimizer / state: as Engine.train_step."""
         eng = self.eng
         assert h_inputs.is_pinned() and h_onehot.is_pinned() and h_inputs.is_contiguous(), "HostFeed needs pinned host tensors"
         a = L.TcrStepArgs()
@@ -334,8 +419,9 @@ class HostFeed:
         if h_clips is not None:
             assert h_clips.is_pinned() and h_clips.dtype == torch.uint8 and h_inputs.dtype == torch.int16
             a.clips, a.background, a.pcm_stride = h_clips.data_ptr(), eng._ptr(background), h_inputs.shape[1]
-        a.params, a.slots, a.moving = eng._ptr(params), eng._ptr(slots), eng._ptr(moving)
-        a.learning_rate, a.momentum, a.weight_decay = float(learning_rate), float(momentum), float(weight_decay)
+        a.params, a.moving = eng._ptr(params), eng._ptr(moving)
+        _set_rule(a, eng._ptr, slots, momentum, optimizer, state)
+        a.learning_rate, a.weight_decay = float(learning_rate), float(weight_decay)
         a.dropout_seed, a.apply_update = int(dropout_seed), 1
         L.check(eng.lib, eng.lib.tcr_train_step_host(eng._h, C.byref(a), self.lag, eng._stream, self._out, C.byref(self._step)),
                 "tcr_train_step_host")

@@ -16,9 +16,13 @@ import torch
 
 from ..common import utils
 from ..datasets import preprocessor_factory
-from ..engine import Engine
+from ..engine import Engine, Optimizer, OptimizerState
 from ..runtime import InvalidArgumentError, Node
 from .base import TFModel
+
+# TF names of the per-variable optimizer state: `<var><suffix>` (slot_creator / ExponentialMovingAverage.average_name)
+SLOT_SUFFIXES = {"mom": ("/Momentum",), "gd": ("/Momentum",), "adam": ("/Adam", "/Adam_1"), "rmsprop": ("/RMSProp", "/RMSProp_1")}
+EMA_SUFFIX = "/ExponentialMovingAverage"
 
 _available_nets = [
     "KWSModel", "Res8Model", "Res8NarrowModel", "Res15Model", "Res15NarrowModel", "DSCNNSModel", "DSCNNMModel",
@@ -34,7 +38,8 @@ class AudioNetModel(TFModel):
         self.args, self.dataset = args, dataset
         self.engine: Optional[Engine] = None
         self.global_step = 0
-        self.optimizer = dict(kind="mom", momentum=0.9)            # filled in by the trainer (build_optimizer)
+        self.optimizer = Optimizer("mom", momentum=0.9)             # set by the trainer (build_train_op -> set_optimizer)
+        self.opt_state: Optional[OptimizerState] = None              # its device buffers (Engine.new_optimizer_state)
         self.lr_schedule = lambda step: getattr(args, "learning_rate", 1e-4)
         self.var_names_to_values = None                            # in-memory weight injection hook (trainer.py:145-154)
         self.endpoints_loss: Dict[str, Node] = {}
@@ -87,6 +92,7 @@ class AudioNetModel(TFModel):
                              dropout_keep_prob=a.dropout_keep_prob,
                              label_smoothing=getattr(a, "label_smoothing", 0.0))
         self.params, self.slots, self.moving = self.engine.new_variables(seed=getattr(a, "seed", 0) or 0)
+        self.opt_state = OptimizerState(slots=self.slots)           # momentum until the trainer says otherwise (set_optimizer)
         if getattr(a, "data_parallel", False):
             self.engine.attach_process_group()
         n = int(getattr(a, 'batch_size', 1) or 1)
@@ -140,21 +146,65 @@ class AudioNetModel(TFModel):
     def outputs(self):
         return self._outputs
 
+    # ------------------------------------------------------------------ optimizer state
+    def set_optimizer(self, optimizer: Optimizer):
+        """Adopt the trainer's update rule (helper/trainer.py build_train_op) and create its state the way TF initialises it
+        (Engine.new_optimizer_state); the existing slot buffer becomes its first slot."""
+        self.optimizer = optimizer
+        if self.engine is not None:
+            self.flush_feed()
+            self.opt_state = self.engine.new_optimizer_state(optimizer, self.params, self.slots)
+            self.slots = self.opt_state.slots
+
+    def _state_buffers(self):
+        """(TF variable-name suffix, flat buffer) of every per-variable slot / shadow of the current rule."""
+        st, kind = self.opt_state or OptimizerState(slots=self.slots), self.optimizer.kind
+        out = [(s, b) for s, b in zip(SLOT_SUFFIXES[kind], (st.slots, st.slots2)) if b is not None]
+        if self.optimizer.ema_decay is not None and st.ema is not None:
+            out.append((EMA_SUFFIX, st.ema))
+        return out
+
     # ------------------------------------------------------------------ variables by TF name
     def get_variables(self, with_slots=True) -> Dict[str, np.ndarray]:
+        """Model variables, and with_slots=True the optimizer's state under TF's names: `<var>/Momentum`, `<var>/Adam` +
+        `<var>/Adam_1` + `beta1_power` / `beta2_power`, `<var>/RMSProp` + `<var>/RMSProp_1`, `<var>/ExponentialMovingAverage`."""
         self.flush_feed()
         out = self.engine.variables_to_dict(self.params, self.moving)
         if with_slots:
-            for k, v in self.engine.variables_to_dict(self.slots).items():
-                out[k + "/Momentum"] = v
+            for suffix, buf in self._state_buffers():
+                for k, v in self.engine.variables_to_dict(buf).items():
+                    out[k + suffix] = v
+            st = self.opt_state
+            if self.optimizer.kind == "adam" and st is not None and st.scalars is not None:
+                powers = st.scalars.detach().cpu().numpy()
+                out["beta1_power"], out["beta2_power"] = np.float32(powers[0]).reshape(()), np.float32(powers[1]).reshape(())
         return out
 
     def set_variables(self, values: Dict[str, np.ndarray], strict=True):
+        """Restore by TF name.  Optimizer state the checkpoint does not hold keeps its initial value."""
         self.flush_feed()
         self.engine.variables_from_dict(values, self.params, self.moving, strict=strict)
-        slots = {k[:-len("/Momentum")]: v for k, v in values.items() if k.endswith("/Momentum")}
-        if slots:
-            self.engine.variables_from_dict(slots, self.slots, None, strict=False)
+        for suffix, buf in self._state_buffers():
+            slots = {k[:-len(suffix)]: v for k, v in values.items() if k.endswith(suffix)}
+            if slots:
+                self.engine.variables_from_dict(slots, buf, None, strict=False)
+        st = self.opt_state
+        if self.optimizer.kind == "adam" and st is not None and st.scalars is not None:
+            for i, name in enumerate(("beta1_power", "beta2_power")):
+                if name in values:
+                    st.scalars[i] = float(np.asarray(values[name], np.float32).reshape(()))
+
+    def set_variables_from_ema(self, values: Dict[str, np.ndarray], strict=True):
+        """evaluate_audio.py --use_ema (common/model_loader.py:62-67, ExponentialMovingAverage.variables_to_restore): every
+        trainable from its `<var>/ExponentialMovingAverage` shadow, everything else under its own name."""
+        mapped = dict(values)
+        for d in self.engine.table:
+            if d["trainable"]:
+                mapped.pop(d["name"], None)
+                shadow = d["name"] + EMA_SUFFIX
+                if shadow in values:
+                    mapped[d["name"]] = values[shadow]
+        self.set_variables(mapped, strict=strict)
 
     def _dropout_seed(self):
         """Counter-RNG seed of this step: distinct per rank under data parallelism (the kernel indexes utterances locally)."""
@@ -197,8 +247,8 @@ class AudioNetModel(TFModel):
             from ..engine import HostFeed
             self._feed = HostFeed(self.engine, lag=lag)
         lr = float(self.lr_schedule(self.global_step))
-        r = self._feed.submit(pinned[0], pinned[1], self.params, self.slots, self.moving, lr, self.optimizer.get("momentum") or 0.0,
-                              self.args.weight_decay, dropout_seed=self._dropout_seed())
+        r = self._feed.submit(pinned[0], pinned[1], self.params, self.slots, self.moving, lr, weight_decay=self.args.weight_decay,
+                              dropout_seed=self._dropout_seed(), optimizer=self.optimizer, state=self.opt_state)
         self.global_step += 1
         self._feed_steps.append(self.global_step)
         if r is not None:
@@ -235,8 +285,9 @@ class AudioNetModel(TFModel):
         if "train_op" in names:
             lr = float(self.lr_schedule(self.global_step))
             out = self.engine.train_step(self._d_wav, self._d_hot, self.params, self.slots, self.moving, lr,
-                                         self.optimizer.get("momentum") or 0.0, wd, dropout_seed=self._dropout_seed(),
-                                         want_outputs=bool(names & {"outputs", "logits"}))
+                                         weight_decay=wd, dropout_seed=self._dropout_seed(),
+                                         want_outputs=bool(names & {"outputs", "logits"}), optimizer=self.optimizer,
+                                         state=self.opt_state)
             self.global_step += 1
             vals["train_op"], vals["learning_rate"] = None, np.float32(lr)
         else:

@@ -34,7 +34,11 @@ class Evaluator:
     def evaluate_once(self, checkpoint_path):
         self.log.info("Evaluation started")
         self.setup_dataset_iterator()
-        self.model.set_variables(ckpt.load(checkpoint_path), strict=not self.args.ignore_missing_vars)
+        values = ckpt.load(checkpoint_path)
+        if getattr(self.args, "use_ema", False):       # trainables from their EMA shadows (common/model_loader.py:62-67)
+            self.model.set_variables_from_ema(values, strict=not self.args.ignore_missing_vars)
+        else:
+            self.model.set_variables(values, strict=not self.args.ignore_missing_vars)
         step = self.build_evaluation_step(str(checkpoint_path))
         self.model.global_step = step
         metrics = self.run_evaluation(step, is_training=False)

@@ -2,18 +2,22 @@
 
 What changes underneath: `build_train_op` does not assemble a gradient graph (slim.learning.create_train_op,
 :199-222) — it arms the model so that fetching the train op in `session.run` executes ONE fused CUDA training step
-(front-end, forward, backward, SGD-momentum, BN moving averages).  The learning rate is
+(front-end, forward, backward, optimizer update, BN moving averages).  The learning rate is
 tf.train.piecewise_constant(global_step, boundaries, lr_list) (:135) evaluated on the host per step.
-Optimizers: "mom" (script default) and "gd" (= momentum 0) run on the CUDA path; "adam"/"rmsprop" raise.
+Optimizers (:171-197): "mom" (the TC-ResNet recipes), "gd" (= momentum 0), "adam" (the CLI default) and "rmsprop" all run in
+the fused step's update kernel; --use_ema adds tf.train.ExponentialMovingAverage(--ema_decay) shadows of the trainables,
+updated in the same kernel after the optimizer (:213-217).
 """
 from __future__ import annotations
 
+import dataclasses
 import sys
 import time
 from pathlib import Path
 
 from ..common import checkpoint as ckpt
 from ..common import utils
+from ..engine import Optimizer
 from ..metrics.manager import AudioMetricManager
 from ..runtime import InvalidArgumentError, Node, no_op
 from .base import AudioBase
@@ -65,23 +69,40 @@ class TrainerBase:
         self.max_to_keep = max_to_keep
 
     def build_optimizer(self, optimizer, learning_rate, momentum=None, decay=None, epsilon=None):
+        """The update rule with its hyper-parameters (engine.Optimizer).  Like the reference, momentum / decay / epsilon are
+        forwarded to the TF optimizer only when truthy, so AdamOptimizer given --momentum or --optimizer_decay raises the same
+        TypeError (it has no such argument); RMSProp takes all three.  "mom" and "gd" ignore the flags they do not use."""
+        kwargs = {}
+        if momentum:
+            kwargs["momentum"] = momentum
+        if decay:
+            kwargs["decay"] = decay
+        if epsilon:
+            kwargs["epsilon"] = epsilon
         if optimizer == "mom":
             self.log.info("Use MomentumOptimizer")
-            return dict(kind="mom", momentum=momentum if momentum is not None else 0.0)
+            return Optimizer("mom", momentum=momentum if momentum is not None else 0.0)
         if optimizer == "gd":
             self.log.info("Use GradientDescentOptimizer")
-            return dict(kind="gd", momentum=0.0)
-        if optimizer in ("adam", "rmsprop"):
-            raise NotImplementedError(f"optimizer '{optimizer}' is not on the CUDA path (TC-ResNet recipes use --optimizer mom)")
+            return Optimizer("gd", momentum=0.0)
+        if optimizer == "adam":
+            for bad in ("momentum", "decay"):
+                if bad in kwargs:
+                    raise TypeError(f"__init__() got an unexpected keyword argument '{bad}'")
+            self.log.info("Use AdamOptimizer")
+            return Optimizer.adam(**kwargs)
+        if optimizer == "rmsprop":
+            self.log.info("Use RMSPropOptimizer")
+            return Optimizer.rmsprop(**kwargs)
         self.log.error(f"Unknown optimizer: {optimizer}")
         raise NotImplementedError
 
     def build_train_op(self, total_loss, optimizer, trainable_scopes, global_step, gradient_multipliers=None):
         if trainable_scopes:
             raise NotImplementedError("--trainable_scopes (partial training) is not supported by the fused step")
-        if self.args.use_ema:
-            raise NotImplementedError("--use_ema is not supported by the fused step")
-        self.model.optimizer = optimizer
+        if getattr(self.args, "use_ema", False):
+            optimizer = dataclasses.replace(optimizer, ema_decay=float(self.args.ema_decay))
+        self.model.set_optimizer(optimizer)
         return Node("train_op")
 
     def routine_restore_and_initialize(self, checkpoint_path=None):
